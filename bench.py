@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Bench of the ProPainter hot path: inpainted frames/s at 640x360 on an 80-frame subvideo (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--mode strong|weak]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--mode strong|weak] [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path (RAFT -> flow completion -> image propagation -> sliding-window
 generator -> composite) over one synthetic 80-frame 640x360 clip.  `value` is measured with the prepared tensors
@@ -19,6 +19,10 @@ git-ignored but travels to the GPU box) on the host cores: one pass over the fir
 threads; it also reports the reference's own PyTorch-CUDA fp16 path on the same B200 at the full 80 frames
 (`reference_cuda`, the number SURVEY.md 8d calls "the number to beat").  Without baseline/_ref it falls back to the
 CPU oracle port.
+
+`--dump-outputs DIR` (b200 arm) writes what the last timed step returned -- the composited uint8 frames [T,H,W,3] --
+as DIR/frames.npy, float32 values of a fixed seeded sample of DUMP_PIXELS pixels (all three channels, pixels in
+ascending flat order), so that two builds can be compared output for output on identical inputs.
 """
 import argparse
 import contextlib
@@ -39,6 +43,7 @@ import torch
 
 T_FRAMES, HEIGHT, WIDTH = 80, 360, 640
 T_CONFIG2 = 240
+DUMP_PIXELS, DUMP_SEED = 1 << 21, 0        # 2M pixels x 3 channels x float32 = 24 MiB
 _OUT_FD = 1
 
 
@@ -102,6 +107,15 @@ class ClockSampler(threading.Thread):
 def synthetic_inputs(T=T_FRAMES):
     from comfyui_propainter_nodes_b200.synthetic import synthetic_clip, synthetic_mask
     return synthetic_clip(T, HEIGHT, WIDTH, 1234), synthetic_mask(T, HEIGHT, WIDTH)
+
+
+def dump_outputs(out_dir, frames):
+    """DIR/frames.npy: float32 [DUMP_PIXELS, 3], the pixels of `frames` ([T,H,W,3]) at fixed seeded positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = frames.reshape(-1, frames.shape[-1])
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(rows.shape[0], min(DUMP_PIXELS, rows.shape[0]), replace=False))
+    sample = rows[torch.from_numpy(idx).to(rows.device)].float().cpu().numpy()
+    np.save(os.path.join(out_dir, "frames.npy"), sample)
 
 
 def synthetic_state_dicts():
@@ -293,8 +307,13 @@ def run_b200(args, rank, world):
         uf, um, flows = PI.process_inpainting(models, ft, fm, md, cfg)
         return PI.feature_propagation_device(models.inpaint_model, uf, um, md, flows, orig_dev, cfg)
 
+    last = [None]       # the output of the latest step, kept only for --dump-outputs
+
     def step():
-        return run_clip(ft, fm, md, orig_dev, cfg)
+        out = run_clip(ft, fm, md, orig_dev, cfg)
+        if args.dump_outputs:
+            last[0] = out
+        return out
 
     def staged():
         """Same work as step() on one GPU, with CUDA events between the stages (reported as stage_ms)."""
@@ -342,6 +361,9 @@ def run_b200(args, rank, world):
     l0 = eng.launch_count
     ms_per_step = timed(step, args.steps)
     launches = (eng.launch_count - l0) // max(args.steps, 1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last[0])
+    last[0] = None
     clips = 1 if (strong or world == 1) else world
     value = clips * T_FRAMES / (ms_per_step / 1000.0)
 
@@ -491,7 +513,11 @@ def main():
     ap.add_argument("--no-config2", action="store_true", help="skip the 240-frame config[2] leg")
     ap.add_argument("--no-ref-cuda", action="store_true", help="reference arm: skip the reference's PyTorch-CUDA leg")
     ap.add_argument("--profile-out", default=None, help="write the full per-kernel table (JSON) here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="b200 arm: write a fixed seeded sample of the last timed step's frames to DIR/frames.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     global _OUT_FD

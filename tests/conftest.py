@@ -15,11 +15,11 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden2():
     """Round-2 fixtures: BASELINE configs and the chunked / outpaint branches (tests/golden/make_golden_r2.py)."""
-    import numpy as np
-    return np.load(os.path.join(ROOT, "tests", "golden", "reference_outputs_r2.npz"))
+    from tests.golden.sampled import Golden
+    return Golden(os.path.join(ROOT, "tests", "golden", "reference_outputs_r2.npz"))
 
 
 @pytest.fixture(scope="session")
 def golden():
-    import numpy as np
-    return np.load(os.path.join(ROOT, "tests", "golden", "reference_outputs.npz"))
+    from tests.golden.sampled import Golden
+    return Golden(os.path.join(ROOT, "tests", "golden", "reference_outputs.npz"))

@@ -1,14 +1,15 @@
 """Round-2 golden fixtures: the reference run on BASELINE.json's configs and on the branches the round-1 cases
-never take (tests/golden/reference_outputs_r2.npz).  Build container only (needs /root/reference):
+never take (tests/golden/reference_outputs_r2.npz).  Needs a checkout of the reference, CPU:
 
-    python tests/golden/make_golden_r2.py
+    python tests/golden/make_golden_r2.py PATH/TO/ComfyUI_ProPainter_Nodes
 
 Like make_golden.py it imports the UNMODIFIED reference (stub ``comfy.model_management``); the two node classes are
 called through their own ``propainter_inpainting`` / ``propainter_outpainting`` methods with
 ``initialize_models`` (which downloads checkpoints) replaced by a function returning the reference's own modules
 loaded with the seeded synthetic checkpoints.  Inputs are regenerated from seeds by the tests; only reference
 OUTPUTS are stored (float32 samples for the RAFT error-growth case, float16 for the other flows -- their
-tolerances are >= 0.02 px and a float16 ulp below 8 px is <= 0.004 px --, uint8 for frames and masks).
+tolerances are >= 0.02 px and a float16 ulp below 8 px is <= 0.004 px --, uint8 for frames and masks).  Masks and
+small arrays are stored whole, frames and flows as fixed samples of their pixels (tests/golden/sampled.py, SPEC below).
 """
 import os
 import sys
@@ -16,22 +17,30 @@ import time
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
-import make_golden as MG  # noqa: E402  (sets up the comfy stub and the reference import)
+import make_golden as MG  # noqa: E402
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
-from reference import propainter_nodes as RN  # noqa: E402
-from reference import propainter_inference as RI  # noqa: E402
-from reference.utils import image_utils as RU  # noqa: E402
-from reference.utils.model_utils import Models  # noqa: E402
-from reference.model.modules.flow_comp_raft import RAFT_bi  # noqa: E402
-
 from comfyui_propainter_nodes_b200 import weights as Wt  # noqa: E402
-from tests.golden import cases  # noqa: E402
+from tests.golden import cases, sampled  # noqa: E402
+
+# sampled arrays: name -> (channel axis, positions); every other output is stored whole
+SPEC = {"c1_image_u8": (3, 4096), "c1_gt_flow_f_s2": (2, 2048), "c1_pred_flow_f": (2, 2048),
+        "chunk_gt_flow_f_s2": (2, 1024), "chunk_pred_flow_f": (2, 2048), "chunk_pred_flow_b": (2, 2048),
+        "chunk_frames_u8": (3, 4096), "outpaint_image_u8": (3, 4096), "outpaint_pred_flow_f": (2, 1024)}
+for _tag in cases.RAFT20_GAINS:
+    SPEC.update({f"raft20_{_tag}_it{it}_s4": (1, 512) for it in cases.RAFT20_ITERS})
+    SPEC[f"raft20_{_tag}_final_s2"] = (1, 1024)
 
 
-def main():
+def main(reference_dir):
+    MG.load_reference(reference_dir)
+    from reference import propainter_nodes as RN
+    from reference import propainter_inference as RI
+    from reference.utils import image_utils as RU
+    from reference.utils.model_utils import Models
+    from reference.model.modules.flow_comp_raft import RAFT_bi
     torch.manual_seed(0)
     torch.set_num_threads(min(16, os.cpu_count() or 1))
     raft, rfc, gen = MG.build_models()
@@ -121,10 +130,10 @@ def main():
     for k, v in out.items():
         a = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
         store[k] = a
-    np.savez_compressed(os.path.join(HERE, "reference_outputs_r2.npz"), **store)
+    np.savez_compressed(os.path.join(HERE, "reference_outputs_r2.npz"), **sampled.shrink(store, SPEC))
     for k, v in store.items():
         print(k, v.shape, v.dtype, float(np.abs(v.astype(np.float64)).mean()))
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

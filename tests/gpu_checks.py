@@ -18,6 +18,7 @@ from comfyui_propainter_nodes_b200.utils import image_utils as IU
 from comfyui_propainter_nodes_b200.utils.model_utils import Models, StageHandle
 from oracle import propainter_oracle as O
 from tests.golden import cases
+from tests.golden.sampled import Golden
 
 DEV = "cuda:0"
 _ENG = {}
@@ -42,6 +43,11 @@ def stats(a, b):
     d = (a - b).abs()
     return dict(max_abs=float(d.max()), mean_abs=float(d.mean()), ref_mean_abs=float(b.abs().mean()),
                 rel=float(d.max() / (b.abs().max() + 1e-12)), nan=bool(torch.isnan(a).any()))
+
+
+def stats_at(golden, k, a):
+    """stats() of the full output `a` against the reference fixture `k`, at the fixture's pixels."""
+    return stats(torch.from_numpy(golden.pick(k, a)), torch.from_numpy(golden[k]))
 
 
 # ------------------------------------------------------------------------------------------------ conv
@@ -194,7 +200,7 @@ def check_raft(golden):
     fr = cases.raft_case()
     ff, fb = m.raft_model.engine.raft_bidir(fr[0].to(DEV), cases.RAFT_ITERS)
     torch.cuda.synchronize()
-    return dict(fwd=stats(ff[None], torch.from_numpy(golden["raft_ff"])), bwd=stats(fb[None], torch.from_numpy(golden["raft_fb"])))
+    return dict(fwd=stats_at(golden, "raft_ff", ff[None]), bwd=stats_at(golden, "raft_fb", fb[None]))
 
 
 def check_rfc(golden):
@@ -202,7 +208,7 @@ def check_rfc(golden):
     (ff, fb), masks = cases.rfc_case()
     of, ob = m.flow_model.engine.flow_complete(ff[0].to(DEV), fb[0].to(DEV), masks[0].to(DEV))
     torch.cuda.synchronize()
-    return dict(fwd=stats(of[None], torch.from_numpy(golden["rfc_f"])), bwd=stats(ob[None], torch.from_numpy(golden["rfc_b"])))
+    return dict(fwd=stats_at(golden, "rfc_f", of[None]), bwd=stats_at(golden, "rfc_b", ob[None]))
 
 
 def check_imgprop(golden):
@@ -210,8 +216,8 @@ def check_imgprop(golden):
     frames, mk, (ff, fb) = cases.imgprop_case()
     uf, um = m.inpaint_model.engine.image_propagate(frames[0].to(DEV), mk[0].to(DEV), ff[0].to(DEV), fb[0].to(DEV))
     torch.cuda.synchronize()
-    d = (uf.cpu() - torch.from_numpy(golden["imgprop_frames"])[0]).abs().max(1).values
-    return dict(frame_mismatch_frac=float((d > 2e-3).float().mean()), frame_max_abs=float(d.max()),
+    d = np.abs(golden.pick("imgprop_frames", uf[None].float()) - golden["imgprop_frames"]).max(1)   # per pixel
+    return dict(frame_mismatch_frac=float((d > 2e-3).mean()), frame_max_abs=float(d.max()),
                 mask_mismatch_frac=float((um.cpu() != torch.from_numpy(golden["imgprop_masks"])[0]).float().mean()))
 
 
@@ -230,7 +236,7 @@ def check_window(golden):
     eng.gen_end()
     torch.cuda.synchronize()
     out = pred[..., :3].permute(0, 3, 1, 2).float()
-    return stats(out[None], torch.from_numpy(golden["window_pred"]))
+    return stats_at(golden, "window_pred", out[None])
 
 
 def check_e2e(golden):
@@ -243,19 +249,20 @@ def check_e2e(golden):
     uf, um, flows = PI.process_inpainting(m, ft, fm, md, cfg)
     comp = PI.feature_propagation(m.inpaint_model, uf, um, md, flows, orig, cfg)
     torch.cuda.synchronize()
-    a, b = np.stack(comp).astype(np.float64), golden["e2e_frames_u8"].astype(np.float64)
+    a, b = golden.pick("e2e_frames_u8", np.stack(comp)).astype(np.float64), golden["e2e_frames_u8"].astype(np.float64)
     mse = ((a - b) ** 2).mean()
-    hole = golden["e2e_masks_dilated"][0, :, 0] > 0.5
+    hole = golden.pick("e2e_frames_u8", golden["e2e_masks_dilated"][0, :, 0] > 0.5)
     mse_hole = (((a - b) ** 2).sum(-1)[hole]).mean() / 3
     return dict(psnr=float(10 * np.log10(255 ** 2 / max(mse, 1e-12))),
                 psnr_hole=float(10 * np.log10(255 ** 2 / max(mse_hole, 1e-12))),
                 max_abs_u8=float(np.abs(a - b).max()), frac_gt1=float((np.abs(a - b) > 1).mean()),
-                flow=stats(flows[0].float(), torch.from_numpy(golden["e2e_pred_flow_f"])),
-                upd_frames=stats(uf.float(), torch.from_numpy(golden["e2e_updated_frames"])))
+                flow=stats_at(golden, "e2e_pred_flow_f", flows[0].float()),
+                upd_frames=stats_at(golden, "e2e_updated_frames", uf.float()))
 
 
 # ------------------------------------------------------------------------------------------------ round 2
 def _psnr_stats(a, b, hole=None):
+    """a, b: [..., 3] uint8 pixels (full frames or the fixture's sampled pixels); hole: [...] bool."""
     a, b = np.asarray(a).astype(np.float64), np.asarray(b).astype(np.float64)
     mse = ((a - b) ** 2).mean()
     out = dict(psnr=float(10 * np.log10(255 ** 2 / max(mse, 1e-12))), max_abs_u8=float(np.abs(a - b).max()),
@@ -286,8 +293,8 @@ def check_c1_node(golden2):
     img, fmask, dmask = ProPainterInpaint().propainter_inpainting(c["image"], c["mask"], **c["kwargs"])
     torch.cuda.synchronize()
     assert img.device.type == "cpu" and img.dtype == torch.float32
-    hole = golden2["c1_masks_dilated_u8"] > 0
-    st = _psnr_stats(_img_u8(img), golden2["c1_image_u8"], hole)
+    hole = golden2.pick("c1_image_u8", golden2["c1_masks_dilated_u8"] > 0)
+    st = _psnr_stats(golden2.pick("c1_image_u8", _img_u8(img)), golden2["c1_image_u8"], hole)
     st["flow_masks_equal"] = bool(np.array_equal(_img_u8(fmask), golden2["c1_flow_masks_u8"]))
     st["masks_dilated_equal"] = bool(np.array_equal(_img_u8(dmask), golden2["c1_masks_dilated_u8"]))
     # stage tensors of the same run
@@ -299,8 +306,8 @@ def check_c1_node(golden2):
                               T, torch.device(DEV), icfg.process_size)
     gt = PI.compute_flow(m.raft_model, ft, cfg)
     uf, um, pf = PI.process_inpainting(m, ft, fm, md, cfg)
-    st["raft_flow"] = stats(gt[0][..., ::2, ::2], torch.from_numpy(golden2["c1_gt_flow_f_s2"]).float())
-    st["pred_flow"] = stats(pf[0], torch.from_numpy(golden2["c1_pred_flow_f"]).float())
+    st["raft_flow"] = stats_at(golden2, "c1_gt_flow_f_s2", gt[0][..., ::2, ::2])
+    st["pred_flow"] = stats_at(golden2, "c1_pred_flow_f", pf[0])
     st["updated_masks_mismatch"] = float((_img_u8(um) != golden2["c1_updated_masks_u8"]).mean())
     return st
 
@@ -315,13 +322,14 @@ def check_raft20(golden2):
         for it in cases.RAFT20_ITERS:
             ff, _ = eng.raft_bidir(fr, it)
             torch.cuda.synchronize()
-            ref = torch.from_numpy(golden2[f"raft20_{tag}_it{it}_s4"])
-            s = stats(ff[:, :, ::4, ::4], ref)
-            d = (ff[:, :, ::4, ::4].cpu() - ref).abs().flatten()
+            k = f"raft20_{tag}_it{it}_s4"
+            got, ref = torch.from_numpy(golden2.pick(k, ff[:, :, ::4, ::4])), torch.from_numpy(golden2[k])
+            s = stats(got, ref)
+            d = (got.float() - ref).abs().flatten()
             s["p99_abs"] = float(torch.quantile(d, 0.99))
             out[f"{tag}_it{it}"] = s
             if it == max(cases.RAFT20_ITERS):
-                out[f"{tag}_final"] = stats(ff[:, :, ::2, ::2], torch.from_numpy(golden2[f"raft20_{tag}_final_s2"]))
+                out[f"{tag}_final"] = stats_at(golden2, f"raft20_{tag}_final_s2", ff[:, :, ::2, ::2])
         eng.close()
     return out
 
@@ -338,11 +346,11 @@ def check_chunked(golden2):
     uf, um, pf = PI.process_inpainting(m, ft, fm, md, cfg)
     comp = PI.feature_propagation(m.inpaint_model, uf, um, md, pf, orig, cfg)
     torch.cuda.synchronize()
-    hole = md[0, :, 0].cpu().numpy() > 0.5
-    st = _psnr_stats(np.stack(comp), golden2["chunk_frames_u8"], hole)
-    st["raft_flow"] = stats(gt[0][..., ::2, ::2], torch.from_numpy(golden2["chunk_gt_flow_f_s2"]).float())
-    st["pred_flow_f"] = stats(pf[0], torch.from_numpy(golden2["chunk_pred_flow_f"]).float())
-    st["pred_flow_b"] = stats(pf[1], torch.from_numpy(golden2["chunk_pred_flow_b"]).float())
+    hole = golden2.pick("chunk_frames_u8", md[0, :, 0].cpu().numpy() > 0.5)
+    st = _psnr_stats(golden2.pick("chunk_frames_u8", np.stack(comp)), golden2["chunk_frames_u8"], hole)
+    st["raft_flow"] = stats_at(golden2, "chunk_gt_flow_f_s2", gt[0][..., ::2, ::2])
+    st["pred_flow_f"] = stats_at(golden2, "chunk_pred_flow_f", pf[0])
+    st["pred_flow_b"] = stats_at(golden2, "chunk_pred_flow_b", pf[1])
     st["updated_masks_mismatch"] = float((_img_u8(um) != golden2["chunk_updated_masks_u8"]).mean())
     return st
 
@@ -353,8 +361,8 @@ def check_outpaint_node(golden2):
     o = cases.outpaint_case()
     img, omask, ow, oh = ProPainterOutpaint().propainter_outpainting(o["image"], **o["kwargs"])
     torch.cuda.synchronize()
-    hole = golden2["outpaint_mask_u8"] > 0
-    st = _psnr_stats(_img_u8(img), golden2["outpaint_image_u8"], hole)
+    hole = golden2.pick("outpaint_image_u8", golden2["outpaint_mask_u8"] > 0)
+    st = _psnr_stats(golden2.pick("outpaint_image_u8", _img_u8(img)), golden2["outpaint_image_u8"], hole)
     st["mask_equal"] = bool(np.array_equal(_img_u8(omask), golden2["outpaint_mask_u8"]))
     st["size_equal"] = [int(ow), int(oh)] == [int(v) for v in golden2["outpaint_size"]]
     return st
@@ -497,8 +505,8 @@ def check_small_workspace_fallback():
 def main():
     import json
     import os
-    golden = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_outputs.npz"))
-    golden2 = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_outputs_r2.npz"))
+    golden = Golden(os.path.join(os.path.dirname(__file__), "golden", "reference_outputs.npz"))
+    golden2 = Golden(os.path.join(os.path.dirname(__file__), "golden", "reference_outputs_r2.npz"))
     only = sys.argv[1:]
     checks = [(f"conv:{n}", (lambda n=n: check_conv(n))) for n in CONV_CASES]
     checks += [("corr_lookup", check_corr_lookup), ("imgprop_step", check_imgprop_step), ("attention", check_attention),

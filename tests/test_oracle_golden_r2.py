@@ -1,8 +1,8 @@
 """Pin the oracle (and the host-side image utilities) to the reference on BASELINE.json's config[0] and on the
 branches the round-1 cases never take: the chunked complete_flow / image_propagation halos and the ref_num window
 schedule (T > subvideo_length), the Outpaint node, 20 RAFT iterations at 640x360.  Fixtures:
-tests/golden/reference_outputs_r2.npz, generated from the unmodified reference by tests/golden/make_golden_r2.py.
-CPU only, fp32."""
+tests/golden/reference_outputs_r2.npz, generated from the unmodified reference by tests/golden/make_golden_r2.py;
+large outputs are compared at the fixture's sampled pixels.  CPU only, fp32."""
 import numpy as np
 import torch
 
@@ -21,9 +21,13 @@ def _sds():
     return SDS
 
 
-def _u8_close(out, ref, frac=2e-3):
-    out, ref = np.asarray(out).astype(np.int32), ref.astype(np.int32)
-    assert out.shape == ref.shape, (out.shape, ref.shape)
+def _max_diff(golden2, k, a):
+    """max |a - reference| over the fixture's pixels of `k` (float16 fixtures compared in float32)."""
+    return float(np.abs(golden2.pick(k, a).astype(np.float32) - golden2[k].astype(np.float32)).max())
+
+
+def _u8_close(golden2, k, out, frac=2e-3):
+    out, ref = golden2.pick(k, np.asarray(out)).astype(np.int32), golden2[k].astype(np.int32)
     bad = (np.abs(out - ref) > 1).mean()
     assert bad < frac, bad
 
@@ -42,12 +46,12 @@ def test_config1_inpaint_node_path(golden2):
     comp, st = O.run_pipeline(*_sds(), ft, fm, md, orig, raft_iter=kw["raft_iter"],
                               subvideo_length=kw["subvideo_length"], neighbor_length=kw["neighbor_length"],
                               ref_stride=kw["ref_stride"], return_stages=True)
-    d = (st["gt_flows"][0][..., ::2, ::2] - torch.from_numpy(golden2["c1_gt_flow_f_s2"]).float()).abs().max()
+    d = _max_diff(golden2, "c1_gt_flow_f_s2", st["gt_flows"][0][..., ::2, ::2])
     assert d < 1e-2, d                      # float16 storage of the fixture: ulp 0.004 below 8 px
-    d = (st["pred_flows"][0] - torch.from_numpy(golden2["c1_pred_flow_f"]).float()).abs().max()
+    d = _max_diff(golden2, "c1_pred_flow_f", st["pred_flows"][0])
     assert d < 1e-2, d
     assert np.array_equal((st["updated_masks"].numpy() * 255).astype(np.uint8), golden2["c1_updated_masks_u8"])
-    _u8_close(np.stack(comp), golden2["c1_image_u8"])
+    _u8_close(golden2, "c1_image_u8", np.stack(comp))
 
 
 def test_raft_20_iterations_640x360(golden2):
@@ -57,9 +61,8 @@ def test_raft_20_iterations_640x360(golden2):
         with torch.no_grad():
             _, trace = O.raft_pairs(sd, fr[0, :-1], fr[0, 1:], max(cases.RAFT20_ITERS), return_trace=True)
         for it in cases.RAFT20_ITERS:
-            ref = torch.from_numpy(golden2[f"raft20_{tag}_it{it}_s4"])
-            d = (trace[it - 1][:, :, ::4, ::4] - ref).abs().max()
-            assert d < 2e-2, (tag, it, float(d))
+            d = _max_diff(golden2, f"raft20_{tag}_it{it}_s4", trace[it - 1][:, :, ::4, ::4])
+            assert d < 2e-2, (tag, it, d)
 
 
 def test_chunked_clip_halos_and_ref_num(golden2):
@@ -71,11 +74,11 @@ def test_chunked_clip_halos_and_ref_num(golden2):
     comp, st = O.run_pipeline(*_sds(), ft, fm, md, orig, raft_iter=e["raft_iter"], subvideo_length=e["subvideo_length"],
                               neighbor_length=e["neighbor_length"], ref_stride=e["ref_stride"], return_stages=True)
     for k, i in (("chunk_pred_flow_f", 0), ("chunk_pred_flow_b", 1)):
-        d = (st["pred_flows"][i] - torch.from_numpy(golden2[k]).float()).abs().max()
-        assert d < 1e-2, (k, float(d))
+        d = _max_diff(golden2, k, st["pred_flows"][i])
+        assert d < 1e-2, (k, d)
     um = (st["updated_masks"].numpy() * 255).astype(np.uint8)
     assert (um != golden2["chunk_updated_masks_u8"]).mean() < 1e-4
-    _u8_close(np.stack(comp), golden2["chunk_frames_u8"])
+    _u8_close(golden2, "chunk_frames_u8", np.stack(comp))
     # the schedule itself: windows of a long clip use <= ref_num + 1 references around the window
     sched = O.window_schedule(e["T"], e["neighbor_length"], e["ref_stride"], e["subvideo_length"])
     assert max(len(r) for _, r in sched) <= e["subvideo_length"] // e["ref_stride"] + 1
@@ -95,6 +98,6 @@ def test_outpaint_node_path(golden2):
     comp, st = O.run_pipeline(*_sds(), ft, fm, md, orig, raft_iter=kw["raft_iter"],
                               subvideo_length=kw["subvideo_length"], neighbor_length=kw["neighbor_length"],
                               ref_stride=kw["ref_stride"], return_stages=True)
-    d = (st["pred_flows"][0] - torch.from_numpy(golden2["outpaint_pred_flow_f"]).float()).abs().max()
+    d = _max_diff(golden2, "outpaint_pred_flow_f", st["pred_flows"][0])
     assert d < 1e-2, d
-    _u8_close(np.stack(comp), golden2["outpaint_image_u8"])
+    _u8_close(golden2, "outpaint_image_u8", np.stack(comp))
